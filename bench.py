@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — exact-GP log-marginal + gradient evaluations per second (fp64), the metric of BASELINE.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 16384] [--d 8]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n 16384] [--d 8] [--dump-outputs DIR]
 
 One "step" = one evaluation (= one GP.parameters_changed(), GPy/core/gp.py:269-282): theta -> log marginal likelihood and
 its gradient w.r.t. (variance, D lengthscales, noise) for GPRegression RBF ARD on the synthetic workload of
@@ -16,6 +16,10 @@ SURVEY.md §8(d) (BASELINE.json configs[1]: N=16384, D=8, fp64, 1xB200).
            is the DMMA GEMM and the peak the DMMA issue rate measured in the same run.
 `cpu_baseline` / `--impl reference`: the reference's own CPU operation sequence (oracle/gpy_oracle.py: same LAPACK/BLAS
            calls incl. the wasted dtrtri, two exp passes, the serial ARD loop compiled from C) on this box's cores.
+`--dump-outputs DIR`: after the timed steps, what the last timed step of each timed path returned to its caller is written
+           as DIR/<name>.npy (float64; the largest, the sparse workload's gradient, has M x D + D + 2 entries). The inputs
+           depend only on the arguments (fixed seeds), so two builds run with the same arguments can be compared output
+           for output.
 """
 import argparse
 import json
@@ -117,6 +121,15 @@ def measured_peaks():
         return 1400.0, "B200_PROFILING.md fallback (1.4 PFLOP/s sustained bf16)"
 
 
+def dump_outputs(args, arrays):
+    """--dump-outputs DIR: each array as DIR/<name>.npy in float64"""
+    if not args.dump_outputs:
+        return
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def dist_env():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -163,23 +176,19 @@ def run_reference(args):
     threads, infos = cpu_threads()
     for w in range(args.warmup):
         cpu_eval_timed(min(N, 2048), D, -1 - w, native)   # warm-up on a small instance: BLAS threads, page cache
-    # Every step is one COMPLETE evaluation at the full size (no extrapolation). One such evaluation takes of the
-    # order of a minute on the host cores, so the run is time-bounded: steps stop once GPX_REF_BUDGET_S (default 240 s)
-    # is spent; at least one step always runs. `steps` in the JSON line is the number actually timed.
-    budget = float(os.environ.get("GPX_REF_BUDGET_S", "240"))
+    # Every step is one COMPLETE evaluation at the full size (no extrapolation); at N = 16384 one takes of the order of a
+    # minute on the host cores.
     times = []
     t_start = time.perf_counter()
     for s in range(args.steps):
         dt, lml, grad = cpu_eval_timed(N, D, s, native)
         times.append(dt)
-        if time.perf_counter() - t_start + dt > budget:
-            break
     total = time.perf_counter() - t_start
     per = float(np.mean(times))
     blas = ", ".join(sorted({"%s %s" % (i.get("internal_api"), i.get("version")) for i in infos}))
     line = {
         "impl": "reference", "metric": METRIC, "value": 1.0 / per, "unit": UNIT, "n_gpus": args.gpus,
-        "steps": len(times), "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": per * 1e3,
+        "steps": len(times), "warmup": args.warmup, "ms_per_step": per * 1e3,
         "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": "GPRegression RBF ARD N=%d D=%d fp64 (BASELINE.json configs[1])" % (N, D),
@@ -189,13 +198,13 @@ def run_reference(args):
                            "dpotri, dpotrs, Cython helpers (symmetrify, serial ARD loop) restated in C, paramz caching "
                            "of r and K modelled"},
         "cpu_baseline": {"value": 1.0 / per, "unit": UNIT, "cores": threads, "kind": "port",
-                         "sample": "%d of %d requested steps, each one complete evaluation at N=%d (time-bounded to %.0f s; "
-                                   "warm-up at N=2048)" % (len(times), args.steps, N, budget),
+                         "sample": "%d steps, each one complete evaluation at N=%d (warm-up at N=2048)" % (len(times), N),
                          "host_cpus": os.cpu_count(), "blas": blas},
         "e2e": {"value": 1.0 / per, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "wall_s": total,
     }
     print(json.dumps(line), flush=True)
+    dump_outputs(args, {"lml": lml, "grad": grad})
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -289,6 +298,10 @@ def run_ours(args):
         e2e_dev_ms.append(eng.stats()["total_ms"])
     barrier()
     e2e_wall = time.perf_counter() - t0
+    if rank == 0:
+        # device-resident path: (log marginal, gradient [variance, lengthscales.., noise], extra jitter) of the last step;
+        # plugin API: log_likelihood() and gradient of its last step
+        dump_outputs(args, {"lml": last[0], "grad": last[1], "jitter": last[2], "e2e_lml": ll, "e2e_grad": g})
     e2e_t = torch.tensor([e2e_wall], dtype=torch.float64, device="cuda")
     if use_dist:
         dist.all_reduce(e2e_t, op=dist.ReduceOp.MAX)
@@ -471,6 +484,7 @@ def run_sparse(args):
         step(i, False)
     torch.cuda.synchronize()
     t_res = time.perf_counter() - t0
+    last = {"lml": m.log_likelihood(), "grad": m.gradient}     # gradient: [Z (M x D, row-major), variance, lengthscales.., noise]
     launches = eng.total_launches() - l0
     clocks = sampler.stop()
     torch.cuda.synchronize()
@@ -479,6 +493,7 @@ def run_sparse(args):
         step(i, True)
     torch.cuda.synchronize()
     t_e2e = time.perf_counter() - t0
+    dump_outputs(args, dict(last, e2e_lml=m.log_likelihood(), e2e_grad=m.gradient))
     flops = 4.0 * N * M * M + 20.0 * M ** 3       # DESIGN.md §7b: tmp, A, dL_dKnm over N M^2 + the M x M algebra
     peak = eng.measure_fp64_peak()
     ach = flops * args.steps / t_res * 1e-12
@@ -526,7 +541,7 @@ def run_sparse(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--size", "--n", dest="n", type=int, default=16384, help="number of data points N")
@@ -538,7 +553,11 @@ def main():
     ap.add_argument("--mode", default="auto", choices=["auto", "sharded", "replicas"],
                     help="N>1 GPUs: auto = independent evaluations per GPU while the matrix fits one GPU (N <= 32768), one "
                          "sharded evaluation beyond; or force either")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "sparse":

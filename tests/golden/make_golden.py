@@ -160,9 +160,31 @@ def main_sparse_het():
         print("%-40s lml %.10f source %s" % (name, lml, source))
 
 
+def main_reference():
+    """tests/golden/reference/: what the reference computes for the inputs of tests/test_reference_crosscheck.py, and the
+    line count of each of its source files (the GPy/...:line citations of include/gpx.h and INTEGRATION.md are checked
+    against it). Needs the reference (GPX_REFERENCE)."""
+    import json
+    sys.path.insert(0, os.path.dirname(HERE))
+    import test_reference_crosscheck as t
+    out = os.path.join(HERE, "reference")
+    os.makedirs(out, exist_ok=True)
+    store = {}
+    G = t.record_reference(store)
+    source = "GPy %s (unmodified, via oracle/paramz_shim)" % G.__version__
+    np.savez_compressed(os.path.join(out, "crosscheck.npz"), source=source, **t.pack(store))
+    with open(os.path.join(out, "gpy_line_counts.json"), "w") as f:
+        json.dump(t.record_line_counts(), f, indent=0)
+        f.write("\n")
+    print("reference numbers of %d arrays, source %s" % (len(store), source))
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "sparse_het":   # only the fixtures added last (the others stay byte-identical)
         main_sparse_het()
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "reference":    # the crosscheck numbers only
+        main_reference()
         sys.exit(0)
     main()
     main_het()
