@@ -8,10 +8,11 @@ from . import _ffi  # noqa: F401
 from ._ffi import Engine, GpxError, kern_K, kern_Kdiag, kern_grad_full  # noqa: F401
 
 from .kern import (RBF, Exponential, Matern32, Matern52, Stationary, DeviceGradient, Add, Prod, White, Bias,  # noqa: F401
-                   Kern, CombinationKernel)
+                   Kern, CombinationKernel, Coregionalize)
 from .inference import (ExactGaussianInference, Gaussian, HeteroscedasticGaussian, MixedNoise,  # noqa: F401
                         PosteriorExact)
-from .model import GP, GPHeteroscedasticRegression, GPRegression  # noqa: F401
+from .model import GP, GPCoregionalizedRegression, GPHeteroscedasticRegression, GPRegression  # noqa: F401
+from .multioutput import ICM, LCM, build_XY  # noqa: F401
 from .sparse import SparseGPRegression, VarDTC  # noqa: F401
 
 __version__ = "0.1.0"

@@ -8,7 +8,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libgpx.so")
 
-KIND = {"rbf": 0, "exponential": 1, "matern32": 2, "matern52": 3, "white": 4, "bias": 5}
+KIND = {"rbf": 0, "exponential": 1, "matern32": 2, "matern52": 3, "white": 4, "bias": 5, "coregionalize": 6}
 GET = {"L": 0, "alpha": 1, "Kinv": 2, "dL_dK": 3, "K": 4, "Linv": 5}
 
 _dp = ctypes.POINTER(ctypes.c_double)
@@ -32,6 +32,11 @@ class GpxKernPart(ctypes.Structure):
                 ("dims", ctypes.POINTER(ctypes.c_int)), ("variance", ctypes.c_double), ("lengthscale", _dp)]
 
 
+class GpxCoreg(ctypes.Structure):
+    """gpx_coreg of include/gpx.h: output_dim and B of one coregionalization part."""
+    _fields_ = [("output_dim", ctypes.c_int), ("B", _dp)]
+
+
 EXPORTS = {
     # name: (restype, argtypes)
     "gpx_last_error": (ctypes.c_char_p, []),
@@ -46,6 +51,8 @@ EXPORTS = {
                                           ctypes.c_int, _dp, _dp, _dp, _dp]),
     "gpx_exact_eval_multi": (ctypes.c_int, [_vp, ctypes.POINTER(GpxKernPart), ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                             ctypes.c_int, _dp, _dp, _dp]),
+    "gpx_exact_eval_coreg": (ctypes.c_int, [_vp, ctypes.POINTER(GpxKernPart), ctypes.c_int, ctypes.POINTER(GpxCoreg),
+                                            ctypes.c_double, _dp, ctypes.c_double, ctypes.c_int, _dp, _dp, _dp, _dp]),
     "gpx_get": (ctypes.c_int, [_vp, ctypes.c_int, _dp]),
     "gpx_predict": (ctypes.c_int, [_vp, _dp, ctypes.c_int64, ctypes.c_int, _dp, _dp]),
     "gpx_kern_K": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_double, _dp, _dp, ctypes.c_int64, _dp,
@@ -214,6 +221,57 @@ class Engine(object):
         self.eval_serial += 1
         check(rc, "gpx_exact_eval_multi")
         return lml.value, grad, jit.value
+
+    def exact_eval_coreg(self, parts, noise, jitter=1e-8, max_tries=5):
+        """composite kernel with coregionalization parts and scalar or per-point noise (gpx_exact_eval_coreg).
+        parts = [(kind, ARD, term, dims, variance, lengthscale)], ordered by term; a "coregionalize" part carries its
+        O x O matrix B in place of the lengthscale and one dim (the output-index column). noise: a float or N variances.
+        -> (log_marginal, gradient [per part: variance, lengthscale.. (none for white / bias) or S (O*O, row-major);
+        then noise], dnoise (N,) or None, extra_jitter)"""
+        arr = (GpxKernPart * len(parts))()
+        co = []
+        keep, ngrad = [], 1
+        for i, (kind, ard, term, dims, variance, lengthscale) in enumerate(parts):
+            if kind == "coregionalize":
+                B = np.ascontiguousarray(lengthscale, dtype=np.float64)
+                d = np.ascontiguousarray(np.atleast_1d(dims), dtype=np.int32)
+                if B.ndim != 2 or B.shape[0] != B.shape[1] or d.size != 1:
+                    raise ValueError("part %d: a coregionalization part needs one dim and a square B" % i)
+                keep += [d, B]
+                arr[i].kind, arr[i].ard, arr[i].term, arr[i].ndims = KIND[kind], 0, int(term), 1
+                arr[i].dims = d.ctypes.data_as(ctypes.POINTER(ctypes.c_int))
+                arr[i].variance, arr[i].lengthscale = 1.0, None
+                co.append((B.shape[0], B))
+                ngrad += B.size
+                continue
+            static = kind in ("white", "bias")
+            d = np.ascontiguousarray([] if static else dims, dtype=np.int32)
+            ls = np.ascontiguousarray([1.0] if static else np.atleast_1d(lengthscale), dtype=np.float64).reshape(-1)
+            if not static and ls.size != (d.size if ard else 1):
+                raise ValueError("part %d: lengthscale does not match its active dims" % i)
+            keep += [d, ls]
+            arr[i].kind, arr[i].ard, arr[i].term, arr[i].ndims = KIND[kind], int(bool(ard)), int(term), int(d.size)
+            arr[i].dims = d.ctypes.data_as(ctypes.POINTER(ctypes.c_int))
+            arr[i].variance, arr[i].lengthscale = float(variance), _ptr(ls)
+            ngrad += 1 + (0 if static else ls.size)
+        carr = (GpxCoreg * max(1, len(co)))()
+        for k, (O, B) in enumerate(co):
+            carr[k].output_dim, carr[k].B = int(O), _ptr(B)
+        nv = np.asarray(noise, dtype=np.float64).reshape(-1)
+        vec = nv.size > 1 or np.ndim(noise) > 0
+        if vec:
+            nv = _f64(nv)
+            if nv.size != self.N:
+                raise ValueError("need one noise variance per data point")
+        dnoise = np.zeros(self.N) if vec else None
+        lml, jit = ctypes.c_double(), ctypes.c_double()
+        grad = np.zeros(ngrad)
+        rc = self._L.gpx_exact_eval_coreg(self._h, arr, len(parts), carr, float(nv.mean()) if vec else float(nv[0]),
+                                          _ptr(nv) if vec else None, float(jitter), int(max_tries), ctypes.byref(lml),
+                                          _ptr(grad), _ptr(dnoise), ctypes.byref(jit))
+        self.eval_serial += 1
+        check(rc, "gpx_exact_eval_coreg")
+        return lml.value, grad, dnoise, jit.value
 
     def get(self, which):
         if which == "alpha":

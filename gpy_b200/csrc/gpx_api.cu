@@ -49,6 +49,7 @@ static void free_data(gpx_ctx* c) {
   c->have_kinv = false;
   for (double** mp : {&c->mXsT, &c->msq, &c->mpartials}) { if (*mp) cudaFree(*mp); *mp = nullptr; }
   c->m_cap = 0;
+  c->m_pcap = 0;
   oz_planes_free(c->ozp[0]);
   oz_planes_free(c->ozp[1]);
   oz_planes_free(c->ozpA);
@@ -113,9 +114,9 @@ int gpx_create(int device, gpx_ctx** out) {
   GPX_CUDA(cudaStreamCreateWithPriority(&c->st2, cudaStreamNonBlocking, prio_hi));
   // between the two: the big panel GEMM on st3 must not hold back the small launches of the diagonal-block chain on st2
   GPX_CUDA(cudaStreamCreateWithPriority(&c->st3, cudaStreamNonBlocking, prio_hi < prio_lo - 1 ? prio_hi + 1 : prio_hi));
-  GPX_CUDA(cudaMalloc(&c->res, (MAX_D + 2 * MAX_PARTS + 8) * sizeof(double)));
+  GPX_CUDA(cudaMalloc(&c->res, RES_CAP * sizeof(double)));
   GPX_CUDA(cudaMalloc(&c->info, sizeof(int)));
-  GPX_CUDA(cudaMallocHost(&c->h_res, (MAX_D + 2 * MAX_PARTS + 8) * sizeof(double)));
+  GPX_CUDA(cudaMallocHost(&c->h_res, RES_CAP * sizeof(double)));
   GPX_CUDA(cudaMallocHost(&c->h_info, sizeof(int)));
   {   // keep freed temporaries of the stand-alone calls cached in the device's default pool
     cudaMemPool_t pool;
@@ -148,6 +149,8 @@ int gpx_destroy(gpx_ctx* c) {
   if (c->res) cudaFree(c->res);
   if (c->dNoiseVec) cudaFree(c->dNoiseVec);
   if (c->dDnoise) cudaFree(c->dDnoise);
+  if (c->mB) cudaFree(c->mB);
+  if (c->mflag) cudaFree(c->mflag);
   if (c->info) cudaFree(c->info);
   if (c->h_res) cudaFreeHost(c->h_res);
   if (c->h_info) cudaFreeHost(c->h_info);
@@ -706,20 +709,33 @@ static int eval_once(gpx_ctx* c, double extra_jitter, Recorder& rec) {
   GPX_CUDA(cudaMemsetAsync(c->info, 0, sizeof(int), st));
   if (c->multi) {
     if (c->m_cap != c->Npad) {
-      for (double** mp : {&c->mXsT, &c->msq, &c->mpartials}) { if (*mp) cudaFree(*mp); *mp = nullptr; }
+      for (double** mp : {&c->mXsT, &c->msq}) { if (*mp) cudaFree(*mp); *mp = nullptr; }
       GPX_CUDA(cudaMalloc(&c->mXsT, (size_t)MAX_D * c->Npad * 8));
       GPX_CUDA(cudaMalloc(&c->msq, (size_t)MAX_PARTS * c->Npad * 8));
-      GPX_CUDA(cudaMalloc(&c->mpartials, (size_t)MAX_PARTS * nt * nt * (MAX_D + 2) * 8));
       c->m_cap = c->Npad;
     }
-    GPX_CHECK(launch_prep_multi(c->dX, c->N, c->D, c->Npad, c->mk, c->mXsT, c->msq, st));
+    size_t pneed = 0;
+    for (int q = 0; q < c->mk.nparts; q++) pneed += (size_t)nt * nt * part_nred(c->mk.part[q]);
+    if (c->m_pcap < pneed) {
+      if (c->mpartials) cudaFree(c->mpartials);
+      c->mpartials = nullptr;
+      c->m_pcap = 0;
+      GPX_CUDA(cudaMalloc(&c->mpartials, pneed * 8));
+      c->m_pcap = pneed;
+    }
+    // the composite K-build is one launch: the sweep's first diagonal block must wait for all of it, not for the event a
+    // previous single-kernel evaluation on this context recorded after its first block row
+    c->kfirst_valid = false;
+    GPX_CUDA(cudaMemsetAsync(c->mflag, 0, sizeof(int), st));
+    GPX_CHECK(launch_prep_multi(c->dX, c->N, c->D, c->Npad, c->mk, c->mXsT, c->msq, c->mflag, st));
     c->eval_launches++;
     KBuildMultiParams kb;
     memset(&kb, 0, sizeof(kb));
     kb.rowsT = c->mXsT; kb.ld_rows = c->Npad; kb.sq_rows = c->msq;
     kb.colsT = c->mXsT; kb.ld_cols = c->Npad; kb.sq_cols = c->msq;
     kb.out = c->S; kb.ld = ld; kb.nrows = c->N; kb.ncols = c->N; kb.sym = 1; kb.same = 1;
-    kb.diag_add = (c->noise + c->jitter) + extra_jitter;
+    kb.diag_add = ((c->het ? 0.0 : c->noise) + c->jitter) + extra_jitter;
+    kb.diag_vec = c->het ? c->dNoiseVec : nullptr;
     kb.mk = c->mk;
     const int h = rec.begin(PH_KBUILD);
     GPX_CHECK(launch_kbuild_multi(kb, nt, nt, st));
@@ -785,24 +801,28 @@ static int eval_once(gpx_ctx* c, double extra_jitter, Recorder& rec) {
     FinalizeMultiParams fm;
     memset(&fm, 0, sizeof(fm));
     const int h = rec.begin(PH_LAUUM, 0.0);
+    double* part = c->mpartials;
     for (int q = 0; q < c->mk.nparts; q++) {
-      double* part = c->mpartials + (size_t)q * nt * nt * (MAX_D + 2);
-      const int nred = std::max(1, part_nl(c->mk.part[q])) + 2;
+      const int nred = part_nred(c->mk.part[q]);
       GPX_CUDA(cudaMemsetAsync(part, 0, (size_t)nt * nt * nred * 8, st));
       GradKinvMultiParams gm;
       memset(&gm, 0, sizeof(gm));
       gm.Kinv = c->Kinv; gm.ld = ld; gm.XsT = c->mXsT; gm.sq = c->msq; gm.ldx = c->Npad; gm.alpha = c->dAlpha;
       gm.N = c->N; gm.P = c->P; gm.nt = nt; gm.part = q; gm.want_noise = q == 0; gm.partials = part; gm.mk = c->mk;
+      gm.dnoise_out = (q == 0 && c->het) ? c->dDnoise : nullptr;
       GPX_CHECK(launch_grad_kinv_multi(gm, st));
       c->eval_launches++;
       fm.partials[q] = part;
+      part += (size_t)nt * nt * nred;
     }
     rec.end(h);
     fm.ntiles = (long)nt * nt; fm.logdet_part = c->logdet_part; fm.nt = nt;
     fm.T = oz ? c->dTfw : c->dT; fm.ld = ld; fm.N = c->N; fm.P = c->P; fm.mk = c->mk; fm.res = c->res;
     GPX_CHECK(launch_finalize_multi(fm, st));
     c->eval_launches++;
-    GPX_CUDA(cudaMemcpyAsync(c->h_res, c->res, (MAX_D + 2 * MAX_PARTS + 8) * sizeof(double), cudaMemcpyDeviceToHost, st));
+    int nres = 4;
+    for (int q = 0; q < c->mk.nparts; q++) nres += part_ngrad(c->mk.part[q]);
+    GPX_CUDA(cudaMemcpyAsync(c->h_res, c->res, nres * sizeof(double), cudaMemcpyDeviceToHost, st));
     GPX_CUDA(cudaMemcpyAsync(c->h_info, c->info, sizeof(int), cudaMemcpyDeviceToHost, st));
     c->oz_last = true;   // K^-1 is stored either way
     return 0;
@@ -875,20 +895,49 @@ extern "C" {
 
 }  // extern "C"
 
-// noise_vec == nullptr: homoscedastic (`noise`); else N per-point variances (`noise` = their mean, used by the ladder)
-static int fill_multi(gpx_ctx* c, const gpx_kern_part* parts, int nparts, double* kdiag_total) {
+// coreg: one gpx_coreg per GPX_COREGIONALIZE part (null: no such part allowed). *kdiag_total = Kdiag of the composite kernel
+// when it is the same at every point (no coregionalization part), else unused (composite_kdiag per point)
+static int fill_multi(gpx_ctx* c, const gpx_kern_part* parts, int nparts, const gpx_coreg* coreg, double* kdiag_total) {
   if (!parts || nparts < 1 || nparts > MAX_PARTS) GPX_FAIL("number of kernel parts must be in [1, 8]");
   MultiKern& mk = c->mk;
   memset(&mk, 0, sizeof(mk));
   mk.nparts = nparts;
-  int off = 0;
+  c->m_coreg = false;
+  int off = 0, nco = 0;
   double total = 0.0, prod = 1.0;
   for (int p = 0; p < nparts; p++) {
     const gpx_kern_part& in = parts[p];
     PartDev& pd = mk.part[p];
-    if (in.kind < 0 || in.kind > GPX_BIAS) GPX_FAIL("unknown kernel kind");
-    if (!(in.variance > 0)) GPX_FAIL("variance must be positive");
+    if (in.kind < 0 || in.kind > GPX_COREGIONALIZE) GPX_FAIL("unknown kernel kind");
     if (p > 0 && in.term < parts[p - 1].term) GPX_FAIL("kernel parts must be ordered by term");
+    if (in.kind == GPX_COREGIONALIZE) {
+      if (!coreg) GPX_FAIL("a coregionalization part needs gpx_exact_eval_coreg and its B");
+      const gpx_coreg& cg = coreg[nco++];
+      if (cg.output_dim < 1 || cg.output_dim > MAX_O) GPX_FAIL("output_dim of a coregionalization part must be in [1, 16]");
+      if (!cg.B) GPX_FAIL("null B of a coregionalization part");
+      if (in.ndims != 1 || !in.dims) GPX_FAIL("a coregionalization part has exactly one active dim (the output index)");
+      if (in.dims[0] < 0 || in.dims[0] >= c->D) GPX_FAIL("active dim outside the data");
+      if (off + 1 > MAX_D) GPX_FAIL("the parts' active dims add up to more than 64");
+      pd.kind = GPX_COREGIONALIZE; pd.term = in.term; pd.D = 1; pd.xoff = off; pd.odim = cg.output_dim;
+      pd.variance = 1.0; pd.inv_ls_iso = 1.0;
+      mk.dims[off] = in.dims[0];
+      mk.ls[off] = 1.0;
+      const int O = cg.output_dim;
+      if (c->hB.size() != (size_t)MAX_PARTS * MAX_O * MAX_O) c->hB.assign((size_t)MAX_PARTS * MAX_O * MAX_O, 0.0);
+      // only the lower tiles of K are built and an off-diagonal tile stands for its mirror in the S reduction: B must be
+      // exactly symmetric, as W W^T + diag(kappa) is
+      for (int a = 0; a < O; a++)
+        for (int b = 0; b < O; b++) {
+          if (!std::isfinite(cg.B[a * O + b])) GPX_FAIL("B of a coregionalization part must be finite");
+          if (cg.B[a * O + b] != cg.B[b * O + a]) GPX_FAIL("B of a coregionalization part must be symmetric");
+          c->hB[(size_t)p * MAX_O * MAX_O + a * O + b] = cg.B[a * O + b];
+        }
+      c->m_coreg = true;
+      off += 1;
+      if (p > 0 && in.term != parts[p - 1].term) { total += prod; prod = 1.0; }
+      continue;
+    }
+    if (!(in.variance > 0)) GPX_FAIL("variance must be positive");
     const bool stat = in.kind >= GPX_WHITE;
     if (!stat && (in.ndims < 1 || !in.dims || !in.lengthscale)) GPX_FAIL("a stationary part needs active dims and a lengthscale");
     pd.kind = in.kind; pd.ard = (!stat && in.ard) ? 1 : 0; pd.term = in.term; pd.D = stat ? 0 : in.ndims; pd.xoff = off;
@@ -909,20 +958,63 @@ static int fill_multi(gpx_ctx* c, const gpx_kern_part* parts, int nparts, double
   total += prod;
   mk.sumD = off;
   *kdiag_total = total;
+  if (c->m_coreg) {
+    if (!c->mB) GPX_CUDA(cudaMalloc(&c->mB, (size_t)MAX_PARTS * MAX_O * MAX_O * 8));
+    GPX_CUDA(cudaMemcpyAsync(c->mB, c->hB.data(), (size_t)MAX_PARTS * MAX_O * MAX_O * 8, cudaMemcpyHostToDevice, c->st));
+  }
+  if (!c->mflag) GPX_CUDA(cudaMalloc(&c->mflag, sizeof(int)));
+  mk.B = c->mB;
   return 0;
+}
+
+// Kdiag of the composite kernel at one point x (D columns, output indices already checked): sum over the terms of the
+// product of the parts' Kdiag (add.py:74-79, prod.py:68-76): variance for the stationary / static kinds (stationary.py:170-173,
+// static.py:30-33), B[idx, idx] for a coregionalization part (coregionalize.py:107-108)
+static double composite_kdiag(const gpx_ctx* c, const double* x) {
+  const MultiKern& mk = c->mk;
+  double total = 0.0, prod = 1.0;
+  for (int p = 0; p < mk.nparts; p++) {
+    const PartDev& pd = mk.part[p];
+    if (p > 0 && pd.term != mk.part[p - 1].term) { total += prod; prod = 1.0; }
+    if (pd.kind == GPX_COREGIONALIZE) {
+      const int a = (int)x[mk.dims[pd.xoff]];
+      prod *= c->hB[(size_t)p * MAX_O * MAX_O + (size_t)a * pd.odim + a];
+    } else {
+      prod *= pd.variance;
+    }
+  }
+  return total + prod;
+}
+
+// every output index of the coregionalization parts in the M x D host points X lies in [0, O)
+static bool coreg_indices_ok(const gpx_ctx* c, const double* X, long M) {
+  for (int p = 0; p < c->mk.nparts; p++) {
+    const PartDev& pd = c->mk.part[p];
+    if (pd.kind != GPX_COREGIONALIZE) continue;
+    for (long m = 0; m < M; m++) {
+      const double v = X[m * c->D + c->mk.dims[pd.xoff]];
+      if (!(v > -1.0 && v < (double)pd.odim)) return false;
+    }
+  }
+  return true;
 }
 
 static int exact_eval_impl(gpx_ctx* c, int kind, int ard, double variance, const double* lengthscale, double noise,
                            const double* noise_vec, double jitter, int max_tries, double* lml, double* grad,
-                           double* dnoise, double* jitter_used, const gpx_kern_part* parts = nullptr, int nparts = 0) {
+                           double* dnoise, double* jitter_used, const gpx_kern_part* parts = nullptr, int nparts = 0,
+                           const gpx_coreg* coreg = nullptr) {
   if (!c || !lml || !grad || (!parts && !lengthscale)) GPX_FAIL("null argument");
   if (!c->S) GPX_FAIL("gpx_set_data has not been called");
   if (!(noise >= 0)) GPX_FAIL("noise variance must be non-negative");
   GPX_CUDA(cudaSetDevice(c->device));
+  // the kernel description is rewritten below: a call rejected half-way must not leave the previous posterior usable
+  // with a half-filled kernel (gpx_get(K) / gpx_predict)
+  c->have_eval = false;
+  c->have_kinv = false;
   c->multi = parts != nullptr;
   if (c->multi) {
     if (c->dist) GPX_FAIL("composite kernels are single-GPU");
-    GPX_CHECK(fill_multi(c, parts, nparts, &variance));     // `variance` = Kdiag of the composite kernel (jitter ladder)
+    GPX_CHECK(fill_multi(c, parts, nparts, coreg, &variance));   // `variance` = Kdiag of the composite kernel (jitter ladder)
     c->kp.variance = variance;
   } else
   GPX_CHECK(fill_kp(c->kp, kind, ard, c->D, variance, lengthscale));
@@ -960,8 +1052,21 @@ static int exact_eval_impl(gpx_ctx* c, int kind, int ard, double variance, const
       GPX_CHECK(eval_once(c, extra, rec));
       GPX_CUDA(cudaStreamSynchronize(c->st));
     }
+    if (c->multi && c->m_coreg) {
+      int bad = 0;
+      GPX_CUDA(cudaMemcpy(&bad, c->mflag, sizeof(int), cudaMemcpyDeviceToHost));
+      if (bad) GPX_FAIL("output index of a coregionalization part outside [0, output_dim)");
+    }
     info = *c->h_info;
     if (info == 0) break;
+    if (tries == 1 && c->multi && c->m_coreg) {
+      // the ladder's mean diagonal (util/linalg.py:66-74) with a per-point Kdiag: its mean over the training points
+      std::vector<double> hx((size_t)c->N * c->D);
+      GPX_CUDA(cudaMemcpy(hx.data(), c->dX, hx.size() * 8, cudaMemcpyDeviceToHost));
+      double s = 0.0;
+      for (long i = 0; i < c->N; i++) s += composite_kdiag(c, hx.data() + (size_t)i * c->D);
+      variance = s / (double)std::max<long>(c->N, 1);
+    }
     // jitchol ladder (GPy/util/linalg.py:61-75): the diagonal of Ky is variance + noise + jitter (> 0 here),
     // extra jitter = mean(diag) * 1e-6 * 10^k for k = 0 .. max_tries-1
     if (tries > max_tries) break;
@@ -998,7 +1103,7 @@ static int exact_eval_impl(gpx_ctx* c, int kind, int ard, double variance, const
   *lml = c->h_res[0];
   if (c->multi) {
     int n = 0;
-    for (int p = 0; p < c->mk.nparts; p++) n += 1 + part_nl(c->mk.part[p]);
+    for (int p = 0; p < c->mk.nparts; p++) n += part_ngrad(c->mk.part[p]);
     for (int q = 0; q < n; q++) grad[q] = c->h_res[4 + q];
     grad[n] = c->h_res[3];
   } else
@@ -1025,6 +1130,22 @@ int gpx_exact_eval_multi(gpx_ctx* c, const gpx_kern_part* parts, int nparts, dou
   if (!parts) GPX_FAIL("null argument");
   return exact_eval_impl(c, 0, 0, 1.0, nullptr, noise, nullptr, jitter, max_tries, lml, grad, nullptr, jitter_used, parts,
                          nparts);
+}
+
+int gpx_exact_eval_coreg(gpx_ctx* c, const gpx_kern_part* parts, int nparts, const gpx_coreg* coreg, double noise,
+                         const double* noise_variances, double jitter, int max_tries, double* lml, double* grad,
+                         double* dnoise, double* jitter_used) {
+  if (!c || !parts) GPX_FAIL("null argument");
+  if (!noise_variances) return exact_eval_impl(c, 0, 0, 1.0, nullptr, noise, nullptr, jitter, max_tries, lml, grad, nullptr,
+                                               jitter_used, parts, nparts, coreg);
+  double mean = 0.0;
+  for (int64_t i = 0; i < c->N; i++) {
+    if (!(noise_variances[i] >= 0)) GPX_FAIL("noise variances must be non-negative");
+    mean += noise_variances[i];
+  }
+  mean /= (double)std::max<int64_t>(c->N, 1);
+  return exact_eval_impl(c, 0, 0, 1.0, nullptr, mean, noise_variances, jitter, max_tries, lml, grad, dnoise, jitter_used,
+                         parts, nparts, coreg);
 }
 
 int gpx_exact_eval_het(gpx_ctx* c, int kind, int ard, double variance, const double* lengthscale,
@@ -1411,13 +1532,14 @@ int gpx_predict(gpx_ctx* c, const double* Xnew, int64_t M, int full_cov, double*
   cudaStream_t st = c->st;
   const long ld = c->Npad, N = c->N;
   PointSet pn;
+  if (c->multi && !coreg_indices_ok(c, Xnew, M)) GPX_FAIL("output index of a coregionalization part outside [0, output_dim)");
   if (c->multi) {   // composite kernel: stacked per-part scaled coordinates of the new points
     pn.n = M; pn.ld = (M + TILE - 1) / TILE * TILE; pn.st = c->st;
     GPX_TMP_ALLOC(&pn.raw, (size_t)M * c->D * 8, c->st);
     GPX_TMP_ALLOC(&pn.xT, (size_t)pn.ld * std::max(1, c->mk.sumD) * 8, c->st);
     GPX_TMP_ALLOC(&pn.sq, (size_t)pn.ld * c->mk.nparts * 8, c->st);
     GPX_CUDA(cudaMemcpyAsync(pn.raw, Xnew, (size_t)M * c->D * 8, cudaMemcpyHostToDevice, st));
-    GPX_CHECK(launch_prep_multi(pn.raw, M, c->D, pn.ld, c->mk, pn.xT, pn.sq, st));
+    GPX_CHECK(launch_prep_multi(pn.raw, M, c->D, pn.ld, c->mk, pn.xT, pn.sq, c->mflag, st));
     c->total_launches++;
   } else
   GPX_CHECK(upload_points(c, Xnew, M, c->kp, pn));
@@ -1467,7 +1589,8 @@ int gpx_predict(gpx_ctx* c, const double* Xnew, int64_t M, int full_cov, double*
     if (rc) return rc;
     for (long m = 0; m < M; m++) {
       for (int q = 0; q < c->P; q++) mu[m * c->P + q] = h[(size_t)q * M + m];
-      var[m] = c->kp.variance - h[(size_t)c->P * M + m];
+      // per-point Kdiag of the composite kernel with coregionalization parts, else the one Kdiag of every point
+      var[m] = (c->multi && c->m_coreg ? composite_kdiag(c, Xnew + m * c->D) : c->kp.variance) - h[(size_t)c->P * M + m];
     }
     return 0;
   }
@@ -1518,7 +1641,7 @@ int gpx_predict(gpx_ctx* c, const double* Xnew, int64_t M, int full_cov, double*
     GPX_TMP_ALLOC(&pm.sq, (size_t)pm.ld * c->mk.nparts * 8, c->st);
     GPX_TMP_ALLOC(&dk, (size_t)M * M * 8, c->st);
     GPX_CUDA(cudaMemcpyAsync(pm.raw, Xnew, (size_t)M * c->D * 8, cudaMemcpyHostToDevice, st));
-    rc = launch_prep_multi(pm.raw, M, c->D, pm.ld, c->mk, pm.xT, pm.sq, st);
+    rc = launch_prep_multi(pm.raw, M, c->D, pm.ld, c->mk, pm.xT, pm.sq, c->mflag, st);
     KBuildMultiParams km;
     memset(&km, 0, sizeof(km));
     km.rowsT = pm.xT; km.ld_rows = pm.ld; km.sq_rows = pm.sq; km.colsT = pm.xT; km.ld_cols = pm.ld; km.sq_cols = pm.sq;

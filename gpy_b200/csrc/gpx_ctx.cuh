@@ -93,8 +93,13 @@ struct gpx_ctx {
   gpx::MultiKern mk{};
   double* mXsT = nullptr;      // [sumD][Npad] stacked scaled inputs of the parts
   double* msq = nullptr;       // [nparts][Npad]
-  double* mpartials = nullptr; // [MAX_PARTS][nt*nt][MAX_D+2]
-  long m_cap = 0;              // Npad the three buffers were sized for
+  double* mpartials = nullptr; // per part [nt*nt][part_nred], parts back to back
+  long m_cap = 0;              // Npad the XsT / sq buffers were sized for
+  size_t m_pcap = 0;           // doubles in mpartials: nt*nt * sum over the parts of part_nred
+  bool m_coreg = false;        // the kernel has coregionalization parts (gpx_exact_eval_coreg)
+  double* mB = nullptr;        // [MAX_PARTS][MAX_O * MAX_O] B of the coregionalization parts (MultiKern::B)
+  std::vector<double> hB;      // host copy of mB (composite Kdiag of the jitter ladder and of gpx_predict)
+  int* mflag = nullptr;        // set by prep_multi: an output index outside [0, O)
   struct DistState* dist = nullptr;   // multi-GPU state (gpx_dist.cu), null on a single GPU
   struct SparseState* sparse = nullptr;   // sparse-GP (VarDTC) state (gpx_sparse.cu)
 };

@@ -129,6 +129,9 @@ def _make_combination(base, is_prod):
             if isinstance(dL_dK, DeviceGradient) and X2 is None and dL_dK.part_grads is not None \
                     and dL_dK.matches(_composite_key(self)):
                 for (leaf, _), g in zip(_flatten(self), dL_dK.part_grads):
+                    if getattr(leaf, "_gpx_coreg", False):
+                        _set_coreg_gradients(leaf, g)
+                        continue
                     leaf.variance.gradient = g[0]
                     if hasattr(leaf, "lengthscale"):
                         leaf.lengthscale.gradient = g[1:] if leaf.ARD else g[1]
@@ -140,8 +143,42 @@ def _make_combination(base, is_prod):
     return B200Combination
 
 
+def _set_coreg_gradients(leaf, S):
+    """coregionalize.py:123-128 from the device's S[a, b] = sum of dL_dK over rows of output a and columns of output b"""
+    S = np.array(S, dtype=np.float64).reshape(leaf.output_dim, leaf.output_dim)
+    dkappa = np.diag(S).copy()
+    S += S.T
+    leaf.W.gradient = (np.asarray(leaf.W)[:, None, :] * S[:, :, None]).sum(0)
+    leaf.kappa.gradient = dkappa
+
+
+def _coreg_B(leaf):
+    """coregionalize.py:80, from the current W and kappa"""
+    W = np.asarray(leaf.W, dtype=np.float64)
+    return np.dot(W, W.T) + np.diag(np.asarray(leaf.kappa, dtype=np.float64))
+
+
+def _make_coregionalize(base):
+    """GPy.kern.Coregionalize whose update_gradients_full takes the O x O reduction S a fused evaluation of this kernel
+    alone already made on the device; any other dL_dK goes to the stock method (coregionalize.py:110-137). K, Kdiag and
+    the rest are the reference's. Inside a sum / product, the plugin Add / Prod hand the leaf its S."""
+
+    class B200Coregionalize(base):
+        _gpx_coreg = True
+
+        def update_gradients_full(self, dL_dK, X, X2=None):
+            if isinstance(dL_dK, DeviceGradient) and X2 is None and dL_dK.part_grads is not None \
+                    and len(dL_dK.part_grads) == 1 and dL_dK.matches(_composite_key(self)):
+                _set_coreg_gradients(self, dL_dK.part_grads[0])
+                return
+            return super(B200Coregionalize, self).update_gradients_full(np.asarray(dL_dK, dtype=np.float64), X, X2)
+
+    B200Coregionalize.__name__ = B200Coregionalize.__qualname__ = base.__name__
+    return B200Coregionalize
+
+
 def _is_leaf(k):
-    return hasattr(k, "_gpx_kind") or type(k).__name__ in ("White", "Bias")
+    return hasattr(k, "_gpx_kind") or getattr(k, "_gpx_coreg", False) or type(k).__name__ in ("White", "Bias")
 
 
 def _flatten(kern):
@@ -165,6 +202,8 @@ def _flatten(kern):
 
 
 def _leaf_descriptor(leaf, term):
+    if getattr(leaf, "_gpx_coreg", False):
+        return ("coregionalize", False, term, np.atleast_1d(leaf.active_dims).astype(int).tolist(), 1.0, _coreg_B(leaf))
     var = float(np.asarray(leaf.variance).reshape(-1)[0])
     if not hasattr(leaf, "_gpx_kind"):
         return (type(leaf).__name__.lower(), False, term, [], var, None)
@@ -176,7 +215,8 @@ def _composite_key(kern):
     fl = _flatten(kern)
     if fl is None:
         return None
-    return tuple((t,) + tuple(repr(x) for x in _leaf_descriptor(leaf, t)) for (leaf, t) in fl)
+    return tuple((t,) + tuple(repr(tuple(x.ravel().tolist()) if isinstance(x, np.ndarray) else x)
+                              for x in _leaf_descriptor(leaf, t)) for (leaf, t) in fl)
 
 
 def _make_vardtc(base, kernel_types, ffi):
@@ -255,14 +295,17 @@ def _make_vardtc(base, kernel_types, ffi):
     return B200VarDTC
 
 
-def make(RBF, Exponential, Matern32, Matern52, ExactGaussianInference, ffi=_ffi, Add=None, Prod=None, VarDTC=None):
+def make(RBF, Exponential, Matern32, Matern52, ExactGaussianInference, ffi=_ffi, Add=None, Prod=None, VarDTC=None,
+         Coregionalize=None):
     """Build the plugin classes on top of the given GPy base classes (Add / Prod optional: composite kernels; VarDTC
-    optional: the sparse model)."""
+    optional: the sparse model; Coregionalize optional: multi-output kernels, fused inside Add / Prod or alone)."""
     kernels = {n: _make_kernel(b, _KINDS[n], ffi) for n, b in
                (("RBF", RBF), ("Exponential", Exponential), ("Matern32", Matern32), ("Matern52", Matern52))}
     kernel_types = tuple(kernels.values())
     if Add is not None and Prod is not None:
         kernels["Add"], kernels["Prod"] = _make_combination(Add, False), _make_combination(Prod, True)
+    if Coregionalize is not None:
+        kernels["Coregionalize"] = _make_coregionalize(Coregionalize)
 
     class B200ExactGaussianInference(ExactGaussianInference):
         """GPy.inference.latent_function_inference.ExactGaussianInference with the fused device evaluation; anything the
@@ -293,7 +336,7 @@ def make(RBF, Exponential, Matern32, Matern52, ExactGaussianInference, ffi=_ffi,
                       Z_tilde=None):
             parts = None
             if mean_function is None and K is None and not isinstance(kern, kernel_types):
-                parts = _flatten(kern) if hasattr(kern, "_gpx_is_prod") else None
+                parts = _flatten(kern) if (hasattr(kern, "_gpx_is_prod") or getattr(kern, "_gpx_coreg", False)) else None
             if parts is None and (mean_function is not None or K is not None or not isinstance(kern, kernel_types)):
                 return super(B200ExactGaussianInference, self).inference(kern, X, likelihood, Y, mean_function,
                                                                          Y_metadata, K, variance, Z_tilde)
@@ -302,28 +345,39 @@ def make(RBF, Exponential, Matern32, Matern52, ExactGaussianInference, ffi=_ffi,
             nvec = np.asarray(variance, dtype=np.float64).reshape(-1)
             het = nvec.size > 1                      # HeteroscedasticGaussian (likelihoods/gaussian.py:347-362)
             if parts is not None:
-                if het:
-                    return super(B200ExactGaussianInference, self).inference(kern, X, likelihood, Y, mean_function,
-                                                                             Y_metadata, K, variance, Z_tilde)
-                # sum / product kernel (add.py, prod.py, static.py): ONE gpx_exact_eval_multi, data resident
+                # sum / product kernel (add.py, prod.py, static.py, coregionalize.py): ONE device call, data resident;
+                # with coregionalization parts or one noise variance per data point (MixedNoise, HeteroscedasticGaussian)
+                # gpx_exact_eval_coreg, else gpx_exact_eval_multi
                 Xc = np.ascontiguousarray(X, dtype=np.float64)
                 Yc = np.ascontiguousarray(Y, dtype=np.float64)
+                if het and nvec.size != Yc.shape[0]:
+                    raise ValueError("heteroscedastic noise needs one variance per data point")
                 if not self._data_key.matches(Xc, Yc):
                     self.engine.set_data(Xc, Yc)
                     self._data_key.remember(Xc, Yc)
-                lml, grad, _ = self.engine.exact_eval_multi([_leaf_descriptor(l, t) for (l, t) in parts], float(nvec[0]),
-                                                            jitter=1e-8, max_tries=5)
+                desc = [_leaf_descriptor(l, t) for (l, t) in parts]
+                coreg = het or any(getattr(l, "_gpx_coreg", False) for (l, _) in parts)
+                if coreg:
+                    lml, grad, dnoise, _ = self.engine.exact_eval_coreg(desc, nvec if het else float(nvec[0]), jitter=1e-8,
+                                                                        max_tries=5)
+                else:
+                    lml, grad, _ = self.engine.exact_eval_multi(desc, float(nvec[0]), jitter=1e-8, max_tries=5)
                 if Z_tilde is not None:
                     lml += Z_tilde
                 pg, i = [], 0
                 for (leaf, _) in parts:
-                    n = 1 + (np.asarray(leaf.lengthscale).size if hasattr(leaf, "lengthscale") else 0)
+                    if getattr(leaf, "_gpx_coreg", False):
+                        n = int(leaf.output_dim) ** 2
+                    else:
+                        n = 1 + (np.asarray(leaf.lengthscale).size if hasattr(leaf, "lengthscale") else 0)
                     pg.append(grad[i:i + n])
                     i += n
                 key = _composite_key(kern)
                 post = PosteriorExact(self.engine, Yc.shape[0], Yc.shape[1], key)
                 dL_dK = DeviceGradient(self.engine, key, None, None, Yc.shape[0], part_grads=pg)
-                return post, lml, {"dL_dK": dL_dK, "dL_dthetaL": grad[-1], "dL_dm": _LazyAlpha(post)}
+                # exact_gaussian_inference.py:72 with mixed_noise.py:38-41 / gaussian.py:358-359
+                dL_dthetaL = likelihood.exact_inference_gradients(dnoise, Y_metadata) if het else grad[-1]
+                return post, lml, {"dL_dK": dL_dK, "dL_dthetaL": dL_dthetaL, "dL_dm": _LazyAlpha(post)}
             noise = None if het else float(nvec[0])
             Xs = np.ascontiguousarray(kern._slice_X(X)[0] if _returns_tuple(kern, X) else kern._slice_X(X),
                                       dtype=np.float64)
@@ -363,4 +417,4 @@ def load():
     import GPy
     from GPy.inference.latent_function_inference import ExactGaussianInference, VarDTC
     return make(GPy.kern.RBF, GPy.kern.Exponential, GPy.kern.Matern32, GPy.kern.Matern52, ExactGaussianInference,
-                Add=GPy.kern.Add, Prod=GPy.kern.Prod, VarDTC=VarDTC)
+                Add=GPy.kern.Add, Prod=GPy.kern.Prod, VarDTC=VarDTC, Coregionalize=GPy.kern.Coregionalize)

@@ -11,7 +11,8 @@ Mirrors (same names, argument meaning, return structure and error behaviour):
 import numpy as np
 
 from . import _ffi
-from .kern import (DeviceGradient, Stationary, White, Bias, composite_state_key, flatten_parts, part_descriptor)
+from .kern import (Coregionalize, DeviceGradient, Stationary, White, Bias, composite_state_key, flatten_parts,
+                   part_descriptor)
 from .param import Param, Parameterized
 
 
@@ -241,9 +242,11 @@ class ExactGaussianInference(object):
         nvec = np.asarray(variance, dtype=np.float64).reshape(-1)
         het = nvec.size > 1                          # HeteroscedasticGaussian: a vector reaches diag.add (:55-56)
         noise = nvec if het else float(nvec[0])
-        if mean_function is None and K is None and not het and not isinstance(kern, Stationary):
+        if mean_function is None and K is None and not isinstance(kern, Stationary):
             parts = flatten_parts(kern)
-            if parts is not None:
+            if parts is not None and (het or any(isinstance(k, Coregionalize) for k, _ in parts)):
+                return self._coreg_inference(kern, parts, X, Y, noise, Z_tilde, likelihood, Y_metadata)
+            if parts is not None and not het:
                 return self._composite_inference(kern, parts, X, Y, noise, Z_tilde)
         if mean_function is not None or K is not None or not isinstance(kern, Stationary):
             return self._generic_inference(kern, X, Y, noise, mean_function, K, Z_tilde, likelihood, Y_metadata)
@@ -293,6 +296,32 @@ class ExactGaussianInference(object):
         post = PosteriorExact(self.engine, N, P, key)
         dL_dK = DeviceGradient(self.engine, key, None, None, N, part_grads=part_grads)
         return post, lml, {"dL_dK": dL_dK, "dL_dthetaL": grad[-1], "dL_dm": _LazyAlpha(post)}
+
+    def _coreg_inference(self, kern, parts, X, Y, noise, Z_tilde, likelihood, Y_metadata):
+        """Composite kernels with coregionalization parts (coregionalize.py, util/multioutput.py ICM / LCM) and / or one
+        noise variance per data point (MixedNoise, HeteroscedasticGaussian) on the fused path: ONE gpx_exact_eval_coreg per
+        evaluation. dL_dthetaL = likelihood.exact_inference_gradients(diag(dL_dK)) (exact_gaussian_inference.py:72)."""
+        Xc = np.ascontiguousarray(kern._slice_X(X), dtype=np.float64)
+        Y = np.ascontiguousarray(Y, dtype=np.float64)
+        if np.ndim(noise) > 0 and np.size(noise) != Y.shape[0]:
+            raise ValueError("heteroscedastic noise needs one variance per data point")
+        self._bind(Xc, Y)
+        desc = [part_descriptor(leaf, term) for (leaf, term) in parts]
+        lml, grad, dnoise, _ = self.engine.exact_eval_coreg(desc, noise, jitter=1e-8, max_tries=5)
+        if Z_tilde is not None:
+            lml += Z_tilde
+        part_grads, i = [], 0
+        for (leaf, _) in parts:
+            n = (leaf.output_dim ** 2 if isinstance(leaf, Coregionalize) else
+                 1 + (leaf.lengthscale.size if isinstance(leaf, Stationary) else 0))
+            part_grads.append(grad[i:i + n])
+            i += n
+        N, P = Y.shape
+        key = composite_state_key(kern)
+        post = PosteriorExact(self.engine, N, P, key)
+        dL_dK = DeviceGradient(self.engine, key, None, None, N, part_grads=part_grads)
+        dL_dthetaL = grad[-1] if dnoise is None else likelihood.exact_inference_gradients(dnoise, Y_metadata)
+        return post, lml, {"dL_dK": dL_dK, "dL_dthetaL": dL_dthetaL, "dL_dm": _LazyAlpha(post)}
 
     def _generic_inference(self, kern, X, Y, noise, mean_function, K, Z_tilde, likelihood=None, Y_metadata=None):
         """exact_gaussian_inference.py:37-74 for the cases the fused call does not cover (mean function, precomputed K,

@@ -226,7 +226,7 @@ def flatten_parts(kern):
     """-> list of (leaf kernel, term index) for a kernel that is a leaf, a product of leaves, or a sum of those; None for
     anything else (e.g. a product containing a sum), which then takes the generic inference path."""
     def leaf(k):
-        return isinstance(k, (Stationary, White, Bias))
+        return isinstance(k, (Stationary, White, Bias, Coregionalize))
 
     def product(k, term):
         if leaf(k):
@@ -252,6 +252,8 @@ def part_descriptor(leaf, term):
         return ("white", False, term, [], float(leaf.variance[0]), None)
     if isinstance(leaf, Bias):
         return ("bias", False, term, [], float(leaf.variance[0]), None)
+    if isinstance(leaf, Coregionalize):
+        return ("coregionalize", False, term, leaf.active_dims.tolist(), 1.0, leaf.B)
     kind, ard, var, ls = leaf._theta()
     return (kind, ard, term, leaf.active_dims.tolist(), var, ls)
 
@@ -260,9 +262,9 @@ def composite_state_key(kern):
     fl = flatten_parts(kern)
     if fl is None:
         return None
-    return tuple((t, type(k).__name__, float(k.variance[0]),
-                  tuple(k.lengthscale.values.tolist()) if isinstance(k, Stationary) else (),
-                  tuple(k.active_dims.tolist())) for (k, t) in fl)
+    return tuple((t, type(k).__name__) + (k._state_key() if isinstance(k, Coregionalize) else (
+                  float(k.variance[0]), tuple(k.lengthscale.values.tolist()) if isinstance(k, Stationary) else (),
+                  tuple(k.active_dims.tolist()))) for (k, t) in fl)
 
 
 def scatter_part_gradients(kern, dL_dK):
@@ -271,6 +273,9 @@ def scatter_part_gradients(kern, dL_dK):
     if not (isinstance(dL_dK, DeviceGradient) and dL_dK.part_grads is not None and dL_dK.matches(composite_state_key(kern))):
         return False
     for (leaf, _), g in zip(flatten_parts(kern), dL_dK.part_grads):
+        if isinstance(leaf, Coregionalize):
+            leaf.set_gradients_from_S(np.asarray(g).reshape(leaf.output_dim, leaf.output_dim))
+            continue
         leaf.variance.gradient = np.atleast_1d(g[0])
         if isinstance(leaf, Stationary):
             leaf.lengthscale.gradient = np.atleast_1d(g[1:]).copy()
@@ -425,3 +430,85 @@ class Bias(Static):
 
     def update_gradients_full(self, dL_dK, X, X2=None):
         self.variance.gradient = np.atleast_1d(np.asarray(dL_dK).sum())
+
+
+class Coregionalize(Kern):
+    """GPy.kern.Coregionalize (coregionalize.py:17-157): K(x, x') = B[int(x), int(x')] on one active dim holding the output
+    index, B = W W^T + diag(kappa). W (output_dim x rank) is unconstrained, kappa (output_dim) positive (Logexp). Inside a
+    model evaluated by ExactGaussianInference the part runs on the device (gpx_exact_eval_coreg), which hands back the
+    O x O reduction S of dL_dK; K / Kdiag / update_gradients_full below are the host gathers and sums of the reference for
+    any other caller."""
+
+    def __init__(self, input_dim, output_dim, rank=1, W=None, kappa=None, active_dims=None, name="coregion"):
+        super(Coregionalize, self).__init__(input_dim, active_dims, name)
+        self.output_dim = int(output_dim)
+        self.rank = int(rank)
+        if W is None:                                                          # coregionalize.py:66-69
+            W = 0.5 * np.random.randn(self.output_dim, self.rank) / np.sqrt(self.rank)
+        else:
+            W = np.asarray(W, dtype=np.float64)
+            assert W.shape == (self.output_dim, self.rank)
+        if kappa is None:                                                      # coregionalize.py:71-74
+            kappa = 0.5 * np.ones(self.output_dim)
+        else:
+            kappa = np.asarray(kappa, dtype=np.float64)
+            assert kappa.shape == (self.output_dim,)
+        self.W = Param("W", W, transform=None)
+        self.kappa = Param("kappa", kappa)
+        self.link_parameters(self.W, self.kappa)
+
+    @property
+    def B(self):
+        """coregionalize.py:80"""
+        return np.dot(self.W.values, self.W.values.T) + np.diag(self.kappa.values)
+
+    def _state_key(self):
+        return (tuple(self.W.values.reshape(-1).tolist()), tuple(self.kappa.values.tolist()), tuple(self.active_dims.tolist()))
+
+    def _index(self, X):
+        return np.asarray(self._slice_X(X), dtype=int)[:, 0]
+
+    def K(self, X, X2=None):
+        """coregionalize.py:88-94 (a gather of B)"""
+        i = self._index(X)
+        j = i if X2 is None else self._index(X2)
+        return self.B[i[:, None], j[None, :]]
+
+    def Kdiag(self, X):
+        """coregionalize.py:107-108"""
+        return np.diag(self.B)[self._index(X)]
+
+    def set_gradients_from_S(self, S):
+        """coregionalize.py:123-128 from S[a, b] = sum of dL_dK over rows with index a and columns with index b"""
+        S = np.array(S, dtype=np.float64)
+        dkappa = np.diag(S).copy()
+        S += S.T
+        self.W.gradient = (self.W.values[:, None, :] * S[:, :, None]).sum(0)
+        self.kappa.gradient = dkappa
+
+    def update_gradients_full(self, dL_dK, X, X2=None):
+        """coregionalize.py:110-137 with the NumPy reduction (:130-137)"""
+        i = self._index(X)
+        j = i if X2 is None else self._index(X2)
+        dL_dK = np.asarray(dL_dK, dtype=np.float64)
+        S = np.zeros((self.output_dim, self.output_dim))
+        for a in range(self.output_dim):
+            rows = dL_dK[i == a]
+            for b in range(self.output_dim):
+                S[a, b] = rows[:, j == b].sum()
+        self.set_gradients_from_S(S)
+
+    def update_gradients_diag(self, dL_dKdiag, X):
+        """coregionalize.py:145-151"""
+        i = self._index(X)
+        dL_dKdiag_small = np.array([np.asarray(dL_dKdiag)[i == a].sum() for a in range(self.output_dim)])
+        self.W.gradient = 2. * self.W.values * dL_dKdiag_small[:, None]
+        self.kappa.gradient = dL_dKdiag_small
+
+    def gradients_X(self, dL_dK, X, X2=None):
+        """coregionalize.py:153-154"""
+        return np.zeros(np.asarray(X).shape)
+
+    def gradients_X_diag(self, dL_dKdiag, X):
+        """coregionalize.py:156-157"""
+        return np.zeros(np.asarray(X).shape)

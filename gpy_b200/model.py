@@ -14,7 +14,7 @@ import numpy as np
 
 from .inference import ExactGaussianInference, Gaussian, HeteroscedasticGaussian
 from .kern import RBF
-from .param import Logexp, Parameterized
+from .param import Parameterized
 
 
 class Standardize(object):
@@ -136,13 +136,15 @@ class GP(Parameterized):
 
     @property
     def optimizer_array(self):
-        return np.concatenate([Logexp.finv(p.values).reshape(-1) for p in self._free()])
+        return np.concatenate([(p.values if p.transform is None else p.transform.finv(p.values)).reshape(-1)
+                               for p in self._free()])
 
     @optimizer_array.setter
     def optimizer_array(self, x):
         i = 0
         for p in self._free():
-            p.values[...] = Logexp.f(x[i:i + p.size]).reshape(p.values.shape)
+            v = x[i:i + p.size]
+            p.values[...] = (v if p.transform is None else p.transform.f(v)).reshape(p.values.shape)
             i += p.size
         self.parameters_changed()
 
@@ -157,7 +159,8 @@ class GP(Parameterized):
     def _grads_transformed(self):
         g = []
         for p in self._free():
-            g.append(np.asarray(p.gradient, dtype=np.float64).reshape(-1) * Logexp.gradfactor(p.values).reshape(-1))
+            gf = 1.0 if p.transform is None else p.transform.gradfactor(p.values).reshape(-1)   # W of Coregionalize: none
+            g.append(np.asarray(p.gradient, dtype=np.float64).reshape(-1) * gf)
         return -np.concatenate(g)
 
     def _objective_and_grad(self, x):
@@ -274,3 +277,23 @@ class GPRegression(GP):
         super(GPRegression, self).__init__(X, Y, kernel, likelihood, mean_function=mean_function, name="GP regression",
                                            device=device, engine=engine, Y_metadata=Y_metadata,
                                            normalizer=False if normalizer is None else normalizer)
+
+
+class GPCoregionalizedRegression(GP):
+    """GPy.models.GPCoregionalizedRegression (gp_coregionalized_regression.py:31-46): multi-output regression. X_list /
+    Y_list hold one input / output array per output; the data are stacked with an output-index column (build_XY), the
+    kernel defaults to ICM(RBF) and the likelihood is a MixedNoise of one Gaussian per output. predict() takes the output
+    index as the last column of Xnew and, with include_likelihood, Y_metadata={'output_index': ...} for the noise."""
+
+    def __init__(self, X_list, Y_list, kernel=None, likelihoods_list=None, name="GPCR", W_rank=1, kernel_name="coreg",
+                 device=0, engine=None):
+        from . import multioutput
+        X, Y, self.output_index = multioutput.build_XY(X_list, Y_list)             # :34
+        Ny = len(Y_list)
+        if kernel is None:                                                           # :38-41
+            kernel = RBF(X.shape[1] - 1)
+            kernel = multioutput.ICM(input_dim=X.shape[1] - 1, num_outputs=Ny, kernel=kernel, W_rank=W_rank,
+                                     name=kernel_name)
+        likelihood = multioutput.build_likelihood(Y_list, self.output_index, likelihoods_list)   # :43
+        super(GPCoregionalizedRegression, self).__init__(X, Y, kernel, likelihood, name=name, device=device, engine=engine,
+                                                         Y_metadata={"output_index": self.output_index})

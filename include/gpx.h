@@ -32,7 +32,8 @@ extern "C" {
 typedef struct gpx_ctx gpx_ctx;
 
 enum { GPX_RBF = 0, GPX_EXPONENTIAL = 1, GPX_MATERN32 = 2, GPX_MATERN52 = 3,
-       GPX_WHITE = 4, GPX_BIAS = 5 /* static parts of a composite kernel only (GPy/kern/src/static.py:63-99,142-185) */ };
+       GPX_WHITE = 4, GPX_BIAS = 5, /* static parts of a composite kernel only (GPy/kern/src/static.py:63-99,142-185) */
+       GPX_COREGIONALIZE = 6        /* coregionalization part, gpx_exact_eval_coreg only (GPy/kern/src/coregionalize.py:82-137) */ };
 
 /* gpx_get selectors */
 enum {
@@ -88,16 +89,42 @@ int gpx_exact_eval_het(gpx_ctx* ctx, int kind, int ard, double variance, const d
  *         White / Bias)], then d/d noise — the order paramz gives Add/Prod parameters (kern.py:363-451 link order).
  * gpx_get / gpx_predict afterwards use the composite kernel. Single-GPU. */
 typedef struct {
-  int kind;                  /* GPX_RBF .. GPX_MATERN52, GPX_WHITE, GPX_BIAS */
+  int kind;                  /* GPX_RBF .. GPX_MATERN52, GPX_WHITE, GPX_BIAS (GPX_COREGIONALIZE: gpx_exact_eval_coreg) */
   int ard;                   /* stationary kinds: 0 -> lengthscale points at 1 double, 1 -> at ndims doubles */
   int term;                  /* additive term this factor belongs to */
-  int ndims;                 /* number of active dims (0 for White / Bias) */
+  int ndims;                 /* number of active dims (0 for White / Bias, 1 for a coregionalization part) */
   const int* dims;           /* column indices into X, ndims entries */
   double variance;
   const double* lengthscale;
 } gpx_kern_part;
 int gpx_exact_eval_multi(gpx_ctx* ctx, const gpx_kern_part* parts, int nparts, double noise, double jitter, int max_tries,
                          double* lml, double* grad, double* jitter_used);
+
+/* Multi-output regression (intrinsic / linear coregionalization: GPy/kern/src/coregionalize.py, GPy/util/multioutput.py:48-135,
+ * GPy/models/gp_coregionalized_regression.py:31-46) on the fused path: gpx_exact_eval_multi with two additions.
+ *  - Parts of kind GPX_COREGIONALIZE. Such a part has one active dim, the output-index column of X (a float column as
+ *    build_XY makes it, multioutput.py:48-67); its value at (x_i, x_j) is B[idx_i, idx_j] with idx = the truncated integer
+ *    (np.asarray(X, dtype=int), coregionalize.py:88-108). B = W W^T + diag(kappa) is formed by the caller
+ *    (coregionalize.py:80) and passed in `coreg`, one entry per GPX_COREGIONALIZE part in part order; the part's `variance`
+ *    and `lengthscale` are ignored (its factor in a product is B itself). An index outside [0, output_dim) makes the call
+ *    return <0 with a message; nothing is read out of bounds.
+ *  - noise_variances: NULL -> the scalar `noise` on the diagonal; else N per-point variances (MixedNoise /
+ *    HeteroscedasticGaussian: exact_gaussian_inference.py:55-56 with a vector), and dnoise (N doubles) receives diag(dL_dK),
+ *    which the likelihood's exact_inference_gradients sums per output (mixed_noise.py:38-41, gaussian.py:358-359).
+ *  grad: concatenation over the parts in the given order of [d/d variance, d/d lengthscale (1 or ndims; none for White /
+ *        Bias)] or, for a GPX_COREGIONALIZE part, S = dL_dK_small (output_dim x output_dim, row-major): S[a][b] = sum over
+ *        idx_i = a, idx_j = b of (dL_dK o other factors of the term)_ij (coregionalize.py:130-137, prod.py:377-385). The
+ *        caller forms dkappa = diag(S), dW = (S + S^T) W (coregionalize.py:123-128). Last entry: d/d noise (the sum of
+ *        dnoise when noise_variances was given). Every reduction runs in a fixed order: results are bit-identical run to run.
+ *  Caps: output_dim <= 16, nparts <= 8. gpx_get / gpx_predict afterwards use this kernel (gpx_predict checks the indices of
+ *  Xnew as well). Single-GPU. */
+typedef struct {
+  int output_dim;            /* O: B is O x O */
+  const double* B;           /* O x O row-major, finite and exactly symmetric (else the call returns <0) */
+} gpx_coreg;
+int gpx_exact_eval_coreg(gpx_ctx* ctx, const gpx_kern_part* parts, int nparts, const gpx_coreg* coreg, double noise,
+                         const double* noise_variances, double jitter, int max_tries, double* lml, double* grad,
+                         double* dnoise, double* jitter_used);
 
 /* Lazy device->host fetch of N^2 / N*P results of the last gpx_exact_eval (Posterior / grad_dict consumers:
  * GPy/inference/latent_function_inference/posterior.py:21-77; exact_gaussian_inference.py:74). */
